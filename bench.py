@@ -5,10 +5,11 @@
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path, all host cores
     python bench.py --workload df17_aggressive|tiled_64g|snr_sweep ...   # BASELINE.json configs[2..4]
     python bench.py --workload receivers --receivers 256               # SURVEY 8(f) item 4: many receivers, one GPU
+    python bench.py ... --dump-outputs DIR                              # also write what the last timed step computed to DIR/*.npy
 
-Default workload (BASELINE.json configs[1]): testfiles/modes1.bin tiled back to back to 1 GiB
-(536 870 912 samples = 4096 reference buffers) per GPU, --no-fix.  Weak scaling: rank r holds the
-r-th GiB of the tiled stream.  A step = one pass of the hot path over the rank's GiB:
+Default workload (BASELINE.json configs[1]): a synthetic stand-in for testfiles/modes1.bin (its length,
+seeded) tiled back to back to 1 GiB (536 870 912 samples = 4096 reference buffers) per GPU, --no-fix.
+Weak scaling: rank r holds the r-th GiB of the tiled stream.  A step = one pass of the hot path over the rank's GiB:
   value : inputs resident in HBM; scan + frame-evaluation kernels, every rank on its own shard with
           its outputs in its own HBM (no data-path collective); CUDA events on the launching stream,
           max over ranks.
@@ -44,23 +45,23 @@ METRIC = "Msamples/s (2 MHz u8 IQ) decoded, whole job"
 
 WORKLOADS = {
     # name: (description, decoder flags, bytes per GPU and step, device batches per step)
-    "tiled_nofix": dict(desc="modes1.bin tiled to 1 GiB per GPU, --no-fix (BASELINE.json configs[1])", flags="--no-fix",
+    "tiled_nofix": dict(desc="synthetic stand-in for modes1.bin tiled to 1 GiB per GPU, --no-fix (BASELINE.json configs[1])",
+                        flags="--no-fix",
                         cfg=dict(fix_errors=0), nbytes=GIB, batches=1),
     "df17_aggressive": dict(desc="synthetic 2 MHz IQ with injected DF17 (0/1/2/3 flipped bits in turn), 1 GiB per GPU, "
                                  "full path with --aggressive two-bit repair (BASELINE.json configs[2])",
                             flags="--aggressive", cfg=dict(fix_errors=1, aggressive=1), nbytes=GIB, batches=1),
-    "tiled_64g": dict(desc="modes1.bin tiled to 8 GiB per GPU (64 GiB on 8 GPUs), --no-fix, buffer-per-GPU shards "
+    "tiled_64g": dict(desc="synthetic stand-in for modes1.bin tiled to 8 GiB per GPU (64 GiB on 8 GPUs), --no-fix, buffer-per-GPU shards "
                            "(BASELINE.json configs[3])", flags="--no-fix", cfg=dict(fix_errors=0), nbytes=8 * GIB, batches=2),
 }
 
 
 def load_capture() -> tuple[np.ndarray, str]:
-    """The reference's sample capture if it travelled with the repo, else a synthetic stand-in."""
-    for p in (ROOT / "oracle" / "_ref" / "modes1.bin", Path("/root/reference/testfiles/modes1.bin")):
-        if p.exists():
-            return np.fromfile(p, dtype=np.uint8), "modes1.bin tiled"
+    """A synthetic stand-in for the reference's modes1.bin (same length, seeded): the input this
+    benchmark has always used where the capture was not installed, generated, so it is the same
+    wherever the benchmark runs and comparable with earlier builds' results."""
     from dump1090_b200 import synth
-    return synth.random_traffic(356868, 560, seed=1), "synthetic traffic (modes1.bin absent) tiled"
+    return synth.random_traffic(356868, 560, seed=1), "synthetic stand-in for modes1.bin (356 868 samples, seed 1) tiled"
 
 
 def df17_capture() -> tuple[np.ndarray, str]:
@@ -282,6 +283,43 @@ def messages_digest(arr, n: int) -> str:
     return h.hexdigest()
 
 
+DUMP_SAMPLE = 65536           # rows of records / messages written by --dump-outputs (seeded choice when there are more)
+MESSAGE_COLUMNS = ("sample_pos", "msgbits", "msgtype", "crcok", "crc", "errorbit", "phase_corrected")
+
+
+def _sample_rows(n: int) -> np.ndarray:
+    """A fixed, seeded choice of at most DUMP_SAMPLE row indices out of n, in increasing order."""
+    if n <= DUMP_SAMPLE:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+
+
+def dump_outputs(out_dir: Path, cands: np.ndarray, tiles: np.ndarray, messages, n_messages: int) -> None:
+    """What the last timed step computed, as float64 arrays (every value is exact in float64):
+      tile_counts.npy  records per scan tile of the last device batch (all tiles)
+      records.npy      the batch's candidate records in tile order (the order is the stream's; the
+                       array the kernels fill is in tile completion order), sampled: one row per
+                       record = index, t, then per pass msg[14], msgtype, flags, errorbit, nfixed, crc
+      messages.npy     the messages of the last end-to-end step, sampled: index, MESSAGE_COLUMNS, msg[14]
+      counts.npy       [records, messages] before sampling"""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    order = np.concatenate([np.arange(o, o + c) for o, c in tiles] or [np.zeros(0, np.int64)]).astype(np.int64)
+    recs = cands[order]
+    rows = _sample_rows(recs.size)
+    r = recs[rows]
+    p = r["p"]
+    per_pass = [np.concatenate([p[:, k]["msg"], np.stack([p[:, k][f] for f in ("msgtype", "flags", "errorbit", "nfixed", "crc")], 1)], 1)
+                for k in (0, 1)]
+    np.save(out_dir / "tile_counts.npy", tiles["count"].astype(np.float64))
+    np.save(out_dir / "records.npy", np.concatenate([rows[:, None], r["t"][:, None]] + per_pass, 1).astype(np.float64))
+    m = np.ctypeslib.as_array(messages)[:n_messages]
+    rows = _sample_rows(n_messages)
+    m = m[rows]
+    np.save(out_dir / "messages.npy", np.concatenate([rows[:, None], np.stack([m[f] for f in MESSAGE_COLUMNS], 1), m["msg"]], 1)
+            .astype(np.float64))
+    np.save(out_dir / "counts.npy", np.array([recs.size, n_messages], dtype=np.float64))
+
+
 def run_ours(args) -> None:
     import torch
     import torch.distributed as dist
@@ -385,6 +423,7 @@ def run_ours(args) -> None:
     launches = dec.launch_count() - l0
     ktimes = dec.kernel_times_ms()                  # per batch: scan, eval, both, batches
     n_cand = dec.detect_wait()
+    last_records = dec.detect_fetch(bbuf) if args.dump_outputs and rank == 0 else None
     dev_ms, slow_rank = allmax(dev_ms_rank)
     scan_max, scan_rank = allmax(ktimes[0] * nbatch)
     eval_max, eval_rank = allmax(ktimes[1] * nbatch)
@@ -596,6 +635,8 @@ def run_ours(args) -> None:
 
     e2e_steps = args.steps
     e2e_s_rank, e2e_msgs = run_e2e(e2e_steps)
+    if last_records is not None:
+        dump_outputs(Path(args.dump_outputs), *last_records, out_arr, (dec2 if world == 1 else resolver).output_count())
     e2e_s, e2e_slow = allmax(e2e_s_rank)
     if world > 1:
         t = torch.tensor([e2e_msgs], dtype=torch.int64, device=dev)
@@ -878,14 +919,25 @@ def run_receivers(args) -> None:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 30; snr_sweep has its fixed set of points)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="tiled_nofix", choices=list(WORKLOADS) + ["snr_sweep", "receivers"])
     ap.add_argument("--receivers", type=int, default=256, help="receivers: independent streams, one buffer of each per step")
     ap.add_argument("--frames", type=int, default=10000, help="snr_sweep: frames per SNR point (whole job)")
     ap.add_argument("--gpu-resolve", type=int, default=0, help="N=1 e2e: 1 = the order-dependent half on the GPU too (modes_config.gpu_resolve)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0: candidate records, messages) to DIR/*.npy; "
+                         "the decode workloads only (" + ", ".join(WORKLOADS) + "), not snr_sweep or receivers")
     args = ap.parse_args()
+    if args.workload == "snr_sweep" and args.steps is not None:
+        ap.error("snr_sweep times one decode at each of its 17 SNR points: --steps does not apply")
+    if args.steps is None:
+        args.steps = 30
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in WORKLOADS):
+        ap.error(f"--dump-outputs needs the GPU decode workloads ({', '.join(WORKLOADS)})")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "snr_sweep":

@@ -1,15 +1,20 @@
 """ctypes access to the checker libraries (oracle/ and oracle/_ref) for tests.
 
-TEST INFRASTRUCTURE.  Only tests/, __graft_entry__.smoke() and bench.py's CPU
-baseline legs import this.  `libref` (the unmodified reference compiled into
-oracle/_ref/libref.so) exists only where `make -C oracle ref` ran with
-/root/reference present; the prebuilt file travels to the GPU box.
+TEST INFRASTRUCTURE.  Only tests/, __graft_entry__.smoke() and bench.py import
+this.  `libref` (the unmodified reference compiled into oracle/_ref/libref.so)
+exists only where `make -C oracle ref` ran with the reference sources present.
+The tests never need it: what they compare with was recorded from it into
+tests/golden/ (tests/golden/make_reference_answers.py).
 """
 from __future__ import annotations
 
+import atexit
 import ctypes
+import gzip
+import hashlib
 import os
 import subprocess
+import tempfile
 from pathlib import Path
 
 import numpy as np
@@ -98,7 +103,7 @@ def msg_fields(m: Msg, with_pos: bool = False) -> dict:
 def build_oracle() -> None:
     """Compile the CPU restatement (and, where the reference is mounted, oracle/_ref)."""
     subprocess.run(["make", "-C", str(ORACLE_DIR)], check=True, capture_output=True)
-    if REFERENCE_ROOT.exists():
+    if os.path.isdir(REFERENCE_ROOT):                 # False where it is absent or not readable
         subprocess.run(["make", "-C", str(ORACLE_DIR), "ref"], check=True, capture_output=True)
 
 
@@ -111,10 +116,6 @@ def _load(path: Path):
             build_oracle()
         _libs[path] = ctypes.CDLL(str(path))
     return _libs[path]
-
-
-def have_ref() -> bool:
-    return REF_SO.exists() or REFERENCE_ROOT.exists()
 
 
 def oracle_lib():
@@ -200,17 +201,28 @@ def ref_time_phases(data, fix=1, aggressive=0, check_crc=1, loops=1):
     return float(out[0]), float(out[1])
 
 
-def modes1_path() -> Path:
-    """The reference's sample capture (testfiles/modes1.bin).  `make -C oracle ref`
-    copies it to oracle/_ref/ (git-ignored, shipped to the GPU box)."""
-    for p in (ORACLE_DIR / "_ref" / "modes1.bin", REFERENCE_ROOT / "testfiles" / "modes1.bin"):
-        if p.exists():
-            return p
-    raise FileNotFoundError("modes1.bin not found: run `make -C oracle ref` where /root/reference is mounted")
+MODES1_SHA256 = "3a33e16025da8669149c780075950b4e908ca036ea21f9583c113f60d5fb3094"
+_modes1_file = None
 
 
 def modes1() -> np.ndarray:
-    return np.fromfile(modes1_path(), dtype=np.uint8)
+    """The reference's sample capture testfiles/modes1.bin (713 736 bytes), kept gzipped with the tests."""
+    data = np.frombuffer(gzip.decompress((ROOT / "tests" / "golden" / "modes1.bin.gz").read_bytes()), dtype=np.uint8).copy()
+    assert hashlib.sha256(data.tobytes()).hexdigest() == MODES1_SHA256, "tests/golden/modes1.bin.gz is damaged"
+    return data
+
+
+def modes1_path() -> Path:
+    """modes1() as a file, for programs that read a capture (--ifile): written once per process to a
+    temporary file, removed at exit."""
+    global _modes1_file
+    if _modes1_file is None:
+        fd, name = tempfile.mkstemp(suffix="_modes1.bin")
+        with os.fdopen(fd, "wb") as f:
+            f.write(modes1().tobytes())
+        atexit.register(os.unlink, name)
+        _modes1_file = Path(name)
+    return _modes1_file
 
 
 # ---- tracker door of the reference harness (SURVEY.md 8(f) item 3) -----------------------------
@@ -267,6 +279,9 @@ class RefTracker:
         buf = ctypes.create_string_buffer(1 << 20)
         n = self.lib.ref_track_json(int(metric), buf, 1 << 20)
         return buf.raw[:n].decode("latin1")
+
+    def table(self, now_ms, metric=0, max_rows=15):
+        return ref_track_table(now_ms, metric, max_rows)
 
 
 def ref_track_table(now_ms, metric=0, max_rows=15):

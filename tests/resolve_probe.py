@@ -10,7 +10,7 @@ from dump1090_b200 import api, synth
 mib = int(sys.argv[1]) if len(sys.argv) > 1 else 256
 n_sh = int(sys.argv[2]) if len(sys.argv) > 2 else 8
 C.build_oracle()
-src = np.fromfile(ROOT / "oracle/_ref/modes1.bin", dtype=np.uint8)
+src = C.modes1()
 data = synth.tile_to(src, mib << 20)
 t0 = time.time()
 cands = C.oracle_scan_candidates(data, fix=0, cap=4_000_000)

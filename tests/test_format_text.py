@@ -1,17 +1,13 @@
 """CPU (-m "not gpu"): the full message text (SURVEY §8(f) item 1) against the reference binary's
-own stdout, byte for byte.  Messages come from the product's resolver fed with the checker's
-candidate records; the text from modes_format_message()."""
-import subprocess
-import tempfile
-
+own stdout, byte for byte (its sha256, recorded in tests/golden/reference_answers.json).  Messages
+come from the product's resolver fed with the checker's candidate records; the text from
+modes_format_message()."""
 import numpy as np
 import pytest
 
 import checker as C
+import golden_util as G
 from dump1090_b200 import api, synth
-
-REF_BIN = C.ORACLE_DIR / "_ref" / "ref_dump1090"
-needs_ref_bin = pytest.mark.skipif(not (REF_BIN.exists() or C.REFERENCE_ROOT.exists()), reason="oracle/_ref not built")
 
 
 def _product_text(data, fix=1, aggressive=0, check_crc=1):
@@ -23,29 +19,30 @@ def _product_text(data, fix=1, aggressive=0, check_crc=1):
     return "".join(m.text(check_crc) for m in r.take_messages())
 
 
-def _reference_text(data, flags):
-    C.build_oracle()
-    with tempfile.NamedTemporaryFile(suffix=".bin") as f:
-        f.write(data.tobytes())
-        f.flush()
-        return subprocess.run([str(REF_BIN), "--ifile", f.name, *flags], capture_output=True, check=True).stdout.decode("latin1")
+MODES1_FLAGS = [([], {}), (["--aggressive"], dict(aggressive=1)), (["--no-crc-check"], dict(check_crc=0)),
+                (["--no-fix"], dict(fix=0))]
 
 
-@needs_ref_bin
-@pytest.mark.parametrize("flags,kw", [([], {}), (["--aggressive"], dict(aggressive=1)),
-                                       (["--no-crc-check"], dict(check_crc=0)), (["--no-fix"], dict(fix=0))], ids=str)
+@pytest.mark.parametrize("flags,kw", MODES1_FLAGS, ids=str)
 def test_text_equals_reference_on_modes1(flags, kw, checker_libs):
     data = C.modes1()
-    assert _product_text(data, **kw) == _reference_text(data, flags)
+    G.assert_answer(f"text_equals_reference_on_modes1/{' '.join(flags)}", _product_text(data, **kw).encode("latin1"))
 
 
-@needs_ref_bin
-@pytest.mark.parametrize("seed", [51, 52])
+TRAFFIC_SEEDS = [51, 52]
+TRAFFIC_FLAGS = ["--aggressive", "--no-crc-check"]
+
+
+def text_traffic(seed):
+    return synth.random_traffic(400000, 700, seed, amp_range=(30.0, 110.0), max_flips=1)
+
+
+@pytest.mark.parametrize("seed", TRAFFIC_SEEDS)
 def test_text_equals_reference_on_traffic(seed, checker_libs):
     """All DF / extended-squitter kinds the generator emits (ident, surface, airborne, velocity,
     heading, unknown ME types, DF18, address/parity formats)."""
-    data = synth.random_traffic(400000, 700, seed, amp_range=(30.0, 110.0), max_flips=1)
-    assert _product_text(data, aggressive=1, check_crc=0) == _reference_text(data, ["--aggressive", "--no-crc-check"])
+    text = _product_text(text_traffic(seed), aggressive=1, check_crc=0)
+    G.assert_answer(f"text_equals_reference_on_traffic/{seed}", text.encode("latin1"))
 
 
 def test_text_buffer_too_small_is_safe():
@@ -66,22 +63,22 @@ def test_raw_net_line_is_uppercase():
     assert m.raw_line() == "*5d4840d6abcdef;"               # dump1090.c:1325 "%02x"
 
 
-@needs_ref_bin
+_FULL = "8D4B969699155600E87406F5B69F"
+_SHORT = "5D4840D6ABCDEF"
+HEX_LINES = [f"*{_FULL};", f"  *{_FULL};\r\n", f"*{_FULL.lower()};", f"*{_SHORT};", f"\t*{_SHORT};  ", f"*{_FULL}", f"{_FULL};",
+             f"*{_FULL}00;", f"*{_FULL[:-1]};", f"*{_FULL[:-2]}zz;", "*;x", "", "   ", "*", ";", f"* {_FULL};", f"*{_FULL} ;"]
+
+
 def test_hex_line_parser_matches_reference(checker_libs):
     """modes_parse_hex_line accepts / discards exactly the lines decodeHexMessage does, and yields the
-    frame bytes it decodes (full-length frames: the reference leaves missing bytes uninitialised)."""
-    import ctypes
-    ref = C.ref_lib()
-    full = "8D4B969699155600E87406F5B69F"
-    short = "5D4840D6ABCDEF"
-    lines = [f"*{full};", f"  *{full};\r\n", f"*{full.lower()};", f"*{short};", f"\t*{short};  ", f"*{full}", f"{full};",
-             f"*{full}00;", f"*{full[:-1]};", f"*{full[:-2]}zz;", "*;x", "", "   ", "*", ";", f"* {full};", f"*{full} ;"]
-    for line in lines:
-        out = C.Msg()
-        delivered = ref.ref_decode_hex_line(line.encode(), 1, 0, ctypes.byref(out))
+    frame bytes it decodes (full-length frames: the reference leaves missing bytes uninitialised).
+    Recorded per line: [delivered, msgbits, the 14 message bytes] of the reference."""
+    want = G.answer("hex_line_parser_matches_reference")
+    assert len(want) == len(HEX_LINES)
+    for line, (delivered, msgbits, msg_hex) in zip(HEX_LINES, want):
         got = api.parse_hex_line(line)
         assert (got is not None) == bool(delivered), repr(line)
         if got is not None and len(line.strip()) - 2 in (14, 28):
-            nbytes = out.msgbits // 8
+            nbytes = msgbits // 8
             if nbytes * 2 == len(line.strip()) - 2:          # DF length matches what the line supplied
-                assert got[:nbytes] == bytes(out.msg[:nbytes]), repr(line)
+                assert got[:nbytes] == bytes.fromhex(msg_hex)[:nbytes], repr(line)

@@ -1,5 +1,4 @@
 """-m gpu: edge cases, the hex door, the C host binary, and full-size properties."""
-import ctypes
 import hashlib
 import os
 import subprocess
@@ -9,6 +8,7 @@ import numpy as np
 import pytest
 
 import checker as C
+import golden_util as G
 from dump1090_b200 import api, synth
 
 pytestmark = pytest.mark.gpu
@@ -82,23 +82,27 @@ def test_output_array_equals_callback(gpu_decoder_factory, checker_libs):
     dec.set_output_array(0)
 
 
-@pytest.mark.skipif(not C.have_ref(), reason="needs oracle/_ref")
-def test_hex_door_matches_reference(gpu_decoder_factory, checker_libs):
-    """modes_decode_frame == decodeModesMessage on frame bytes (dump1090.c:2472-2502), incl. repairs."""
+def hex_door_frames():
+    """(aggressive, frame): 120 frames of every DF with 0, 1 or 2 flipped bits, without and then with --aggressive."""
     rng = synth.Counter(7)
-    ref = C.ref_lib()
     for aggressive in (0, 1):
         for k in range(120):
             df = [17, 17, 18, 11, 4, 5, 20, 21, 0, 16][k % 10]
             body = bytes(rng.below(256) for _ in range(10 if df >= 16 else 3))
             frame = synth.flip_bits(synth.make_frame(df, rng.below(8), body), [rng.below(56) for _ in range(k % 3)])
-            frame = frame.ljust(14, b"\0")
-            dec = gpu_decoder_factory(aggressive=aggressive)      # fresh ICAO cache, like the harness
-            want = C.Msg()
-            ref.ref_decode_bytes(frame, 1, aggressive, ctypes.byref(want))
-            got = dec.decode_frame(frame)
-            assert C.msg_fields(got) == C.msg_fields(want), (k, aggressive)
-            dec.close()
+            yield aggressive, frame.ljust(14, b"\0")
+
+
+def test_hex_door_matches_reference(gpu_decoder_factory, checker_libs):
+    """modes_decode_frame == decodeModesMessage on frame bytes (dump1090.c:2472-2502), incl. repairs.
+    The reference's msg_fields of every frame are recorded in tests/golden/reference_answers.json."""
+    got = []
+    for aggressive, frame in hex_door_frames():
+        dec = gpu_decoder_factory(aggressive=aggressive)          # fresh ICAO cache, like the harness
+        got.append(C.msg_fields(dec.decode_frame(frame)))
+        dec.close()
+    assert len(got) == 240
+    G.assert_answer("hex_door_matches_reference", got)
 
 
 def test_hex_door_batch_equals_single_frames(gpu_decoder_factory, checker_libs):
@@ -121,6 +125,9 @@ def test_hex_door_batch_equals_single_frames(gpu_decoder_factory, checker_libs):
         assert any(m["crcok"] for m in got if m["msgtype"] in (4, 5, 20))     # address/parity replies validated by the carried cache
 
 
+C_HOST_TEXT_FLAGS = [[], ["--aggressive", "--no-crc-check"], ["--onlyaddr"]]
+
+
 def test_c_host_binary(checker_libs):
     """./dump1090-b200 --ifile modes1.bin --raw prints the reference's lines (SURVEY.md §4 md5 pins)."""
     exe = ROOT / "dump1090-b200"
@@ -133,17 +140,11 @@ def test_c_host_binary(checker_libs):
         out = subprocess.run([str(exe), "--ifile", f, "--raw", *flags], capture_output=True, check=True).stdout
         assert out.count(b"\n") == n and hashlib.md5(out).hexdigest().startswith(md5), flags
     # default output = the full text of displayModesMessage (dump1090.c:1314-1450): byte-identical to the
-    # reference harness binary, which prints through the reference's own function
-    ref_bin = C.ORACLE_DIR / "_ref" / "ref_dump1090"
-    assert ref_bin.exists(), "oracle/_ref/ref_dump1090 missing: build it with `make oracle` where /root/reference is mounted"
-    if True:
-        for flags in ([], ["--aggressive", "--no-crc-check"]):
-            ours = subprocess.run([str(exe), "--ifile", f, *flags], capture_output=True, check=True).stdout
-            theirs = subprocess.run([str(ref_bin), "--ifile", f, *flags], capture_output=True, check=True).stdout
-            assert ours == theirs, flags
-        ours = subprocess.run([str(exe), "--ifile", f, "--onlyaddr"], capture_output=True, check=True).stdout
-        theirs = subprocess.run([str(ref_bin), "--ifile", f, "--onlyaddr"], capture_output=True, check=True).stdout
-        assert ours == theirs
+    # reference harness binary, which prints through the reference's own function (the sha256 of its
+    # stdout is recorded in tests/golden/reference_answers.json)
+    for flags in C_HOST_TEXT_FLAGS:
+        ours = subprocess.run([str(exe), "--ifile", f, *flags], capture_output=True, check=True).stdout
+        G.assert_answer(f"c_host_binary/{' '.join(flags)}", ours)
     stats = subprocess.run([str(exe), "--ifile", f, "--stats"], capture_output=True, check=True, text=True).stdout
     assert stats.splitlines()[:4] == ["546 valid preambles", "282 demodulated again after phase correction",
                                       "535 demodulated with zero errors", "276 with good crc"]

@@ -30,9 +30,6 @@ def _fields(msgs):
     return [C.msg_fields(m) for m in msgs]
 
 
-needs_ref = pytest.mark.skipif(not C.have_ref(), reason="oracle/_ref not built and /root/reference absent")
-
-
 @pytest.mark.parametrize("kw", FLAG_SETS, ids=str)
 def test_oracle_modes1_pins(kw, checker_libs):
     msgs, _ = C.oracle_decode(C.modes1(), **kw)
@@ -54,24 +51,26 @@ def test_oracle_modes1_stats_pins(checker_libs):
     assert hist == {0: 10, 4: 4, 5: 10, 11: 82, 17: 159, 20: 13, 21: 6}
 
 
-@needs_ref
+# The reference's side of the *_equals_reference tests is recorded in tests/golden/reference_answers.json.
 @pytest.mark.parametrize("kw", FLAG_SETS, ids=str)
 def test_oracle_equals_reference_modes1(kw, checker_libs):
-    r, rs = C.ref_decode(C.modes1(), **kw)
     o, os_ = C.oracle_decode(C.modes1(), **kw)
-    assert _fields(r) == _fields(o)
-    assert rs == os_
+    G.assert_answer(f"oracle_equals_reference_modes1/{kw}", [_fields(o), os_])
 
 
-@needs_ref
-@pytest.mark.parametrize("seed", [11, 12, 13])
-@pytest.mark.parametrize("kw", [dict(), dict(aggressive=1), dict(check_crc=0, aggressive=1)], ids=str)
+SYNTHETIC_SEEDS = [11, 12, 13]
+SYNTHETIC_FLAGS = [dict(), dict(aggressive=1), dict(check_crc=0, aggressive=1)]
+
+
+def synthetic_traffic(seed):
+    return synth.random_traffic(200000 + 7777 * seed, 300, seed, sigma=1.0 + seed % 3)
+
+
+@pytest.mark.parametrize("seed", SYNTHETIC_SEEDS)
+@pytest.mark.parametrize("kw", SYNTHETIC_FLAGS, ids=str)
 def test_oracle_equals_reference_synthetic(seed, kw, checker_libs):
-    data = synth.random_traffic(200000 + 7777 * seed, 300, seed, sigma=1.0 + seed % 3)
-    r, rs = C.ref_decode(data, **kw)
-    o, os_ = C.oracle_decode(data, **kw)
-    assert _fields(r) == _fields(o)
-    assert rs == os_
+    o, os_ = C.oracle_decode(synthetic_traffic(seed), **kw)
+    G.assert_answer(f"oracle_equals_reference_synthetic/{seed}/{kw}", [_fields(o), os_])
 
 
 @pytest.mark.parametrize("name,cid", G.CASES)
@@ -91,14 +90,15 @@ def test_magnitude_pins(checker_libs):
     assert hashlib.sha256(m.astype("<u2").tobytes()).hexdigest().startswith("f116ccd64c38ad15")
 
 
-@needs_ref
-def test_magnitude_equals_reference(checker_libs):
+def magnitude_buffer():
+    """One reference buffer of modes1.bin behind the 476-byte carry, as the reference lays it out."""
     buf = np.full(262620, 127, dtype=np.uint8)
-    d = C.modes1()
-    buf[476: 476 + 262144] = d[:262144]
-    out = np.empty(131310, dtype=np.uint16)
-    C.ref_lib().ref_magnitude(buf.ctypes.data_as(ctypes.c_void_p), out.ctypes.data_as(ctypes.c_void_p))
-    assert np.array_equal(out, C.oracle_magnitude(buf))
+    buf[476: 476 + 262144] = C.modes1()[:262144]
+    return buf
+
+
+def test_magnitude_equals_reference(checker_libs):
+    G.assert_answer("magnitude_equals_reference", C.oracle_magnitude(magnitude_buffer()).astype("<u2"))
 
 
 def test_candidate_pins(checker_libs):
@@ -124,17 +124,12 @@ def test_known_answer_frames(checker_libs):
             assert lib.oracle_checksum(synth.flip_bits(b, [bit]), 112) != 0
 
 
-@needs_ref
 def test_crc_table_matches_reference(checker_libs):
-    # a single set data bit b has checksum == the reference's table entry b
+    # a single set data bit b has checksum == the reference's table entry b (its checksum of
+    # the 112-bit message with only data bit b set)
     tab = (ctypes.c_uint32 * 112)()
     C.oracle_lib().oracle_crc_table(tab)
-    ref = C.ref_lib()
-    ref.ref_checksum.restype = ctypes.c_uint32
-    for b in range(88):
-        msg = bytearray(14)
-        msg[b >> 3] = 0x80 >> (b & 7)
-        assert ref.ref_checksum(bytes(msg), 112) == tab[b]
+    assert G.answer("crc_table_matches_reference") == list(tab[:88])
     assert tab[87] == 0xFFF409 and all(tab[b] == 0 for b in range(88, 112))
 
 
@@ -154,18 +149,30 @@ def test_magnitude_is_strictly_monotone_in_squared_amplitude(checker_libs):
     assert max(ms) == 65167
 
 
-@needs_ref
-def test_decode_bytes_matches_reference(checker_libs):
+def decode_bytes_frames():
+    """300 frames of every DF, 0, 1 or 2 bits flipped, padded to 14 bytes."""
     rng = synth.Counter(99)
-    ref, orc = C.ref_lib(), C.oracle_lib()
     for k in range(300):
         df = [17, 17, 18, 11, 4, 5, 20, 21, 0, 16][k % 10]
         body = bytes(rng.below(256) for _ in range(10 if df >= 16 else 3))
         frame = synth.make_frame(df, rng.below(8), body)
         flips = [rng.below(len(frame) * 8) for _ in range(k % 3)]
-        frame = synth.flip_bits(frame, flips).ljust(14, b"\0")
+        yield synth.flip_bits(frame, flips).ljust(14, b"\0")
+
+
+def decode_bytes_fields(lib, fname):
+    """msg_fields of every frame of decode_bytes_frames() decoded by lib.fname, without and with --aggressive."""
+    fn = getattr(lib, fname)
+    out = []
+    for frame in decode_bytes_frames():
         for aggressive in (0, 1):
-            a, b = C.Msg(), C.Msg()
-            ref.ref_decode_bytes(frame, 1, aggressive, ctypes.byref(a))
-            orc.oracle_decode_bytes(frame, 1, aggressive, ctypes.byref(b))
-            assert C.msg_fields(a) == C.msg_fields(b)
+            m = C.Msg()
+            fn(frame, 1, aggressive, ctypes.byref(m))
+            out.append(C.msg_fields(m))
+    return out
+
+
+def test_decode_bytes_matches_reference(checker_libs):
+    got = decode_bytes_fields(C.oracle_lib(), "oracle_decode_bytes")
+    assert len(got) == 600
+    G.assert_answer("decode_bytes_matches_reference", got)
