@@ -548,7 +548,13 @@ class Resolver:
 class ReceiverPool:
     """modes_pool_*: independent 2 MHz streams (one address cache, carry, skip state and set of
     statistics each, as one dump1090 process keeps per receiver), one buffer of each decoded per
-    batch.  Messages are collected per receiver (`take(receiver)`)."""
+    batch.  Messages are collected per receiver (`take(receiver)`).
+
+    gpu_resolve=1 (a make_config field, like fix_errors): the order-dependent half (skip / retry,
+    address caches, statistics) runs on the device at collect(), one warp per receiver with every
+    receiver's cache resident in device memory, and only the delivered messages' 40-byte records come
+    back.  The output is the same as with gpu_resolve=0, byte for byte; resolve() (the host half alone)
+    is then refused."""
 
     def __init__(self, n_receivers: int, max_batch: int = 0, **cfg):
         self.cfg = make_config(**cfg)

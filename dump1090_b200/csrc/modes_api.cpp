@@ -141,8 +141,10 @@ unsigned event_flags(bool timing) {
     return (timing ? 0u : (unsigned)cudaEventDisableTiming) | (host_wait_mode() ? (unsigned)cudaEventBlockingSync : 0u);
 }
 
+}  // namespace
+
 // cudaStreamSynchronize, or its sleeping equivalent (the stream must belong to the current device).
-cudaError_t wait_stream(cudaStream_t st) {
+cudaError_t modes::wait_stream(cudaStream_t st) {
     if (!host_wait_mode()) return cudaStreamSynchronize(st);
     static thread_local cudaEvent_t ev[64] = {};
     int dev = 0;
@@ -155,6 +157,8 @@ cudaError_t wait_stream(cudaStream_t st) {
     if (cudaEventRecord(ev[dev], st) != cudaSuccess) { (void)cudaGetLastError(); return cudaStreamSynchronize(st); }
     return cudaEventSynchronize(ev[dev]);
 }
+
+namespace {
 
 uint32_t default_cand_capacity(uint64_t n_samples) {
     uint64_t c = n_samples / 64 + 4096;
@@ -496,6 +500,13 @@ int run_buffers(modes_ctx *ctx, const uint8_t *host_iq, size_t n_buffers) {
 }
 
 }  // namespace
+
+void modes::detect_results(const modes_ctx *ctx, const modes_candidate **records, const modes_tile **tiles, uint32_t *n_tiles) {
+    const Slot &s = ctx->detect;
+    *records = s.out_records;
+    *tiles = s.out_tiles;
+    *n_tiles = tiles_for((uint64_t)s.n_buffers * kBufSamples);
+}
 
 // ------------------------------------------------------------------- C ABI
 

@@ -1,5 +1,6 @@
 // modes_internal.h — declarations shared by the CUDA kernels (modes_kernels.cu),
-// the host resolve (modes_resolve.cpp) and the C-ABI glue (modes_api.cpp).
+// the host resolve (modes_resolve.cpp), the C-ABI glue (modes_api.cpp) and the
+// receiver pool (modes_pool.cpp).
 // Product code; never includes anything from oracle/.
 #pragma once
 #include <cstddef>
@@ -102,6 +103,24 @@ struct GpuResolve {
 void launch_gpu_resolve(const GpuResolve &g, const modes_candidate *records, const modes_tile *tiles, uint32_t n_tiles,
                         uint32_t n_buffers, int check_crc, int sm_count, cudaStream_t stream);
 
+// The device resolve of a receiver pool (modes_pool.cpp): a batch of n receivers laid out pad, data, pad,
+// data, ...; list entry i owns data buffer 2i+1.  Every receiver's buffer is independent of the others
+// (the skip state restarts at each buffer, and a receiver is listed once per batch), so one warp per
+// entry replays from that receiver's resident cache and writes the cache back: no guessing, no hand-over.
+struct PoolResolve {
+    uint32_t *caches;            // [n_receivers][1024] resident address caches
+    const uint32_t *ids;         // [n] receiver of entry i | kPoolFresh: start from an empty cache
+    uint32_t *n_deliv;           // [n] deliveries of entry i, followed by
+    uint32_t *stats;             //   [n][8] its statistics of this batch
+    uint32_t *offsets;           // [n + 1]
+    uint32_t *flags;             // [4] scratch of resolve_offsets_kernel
+    modes_delivery *out;         // deliveries, entry by entry in list order, each in stream order; t = position
+    uint32_t capacity;           //   inside the receiver's own buffer.  2 x the batch's candidates: cannot overflow
+};
+constexpr uint32_t kPoolFresh = 1u << 31;
+void launch_pool_resolve(const PoolResolve &p, const modes_candidate *records, const modes_tile *tiles, uint32_t n_tiles,
+                         uint32_t n, int check_crc, cudaStream_t stream);
+
 // ---- sequential resolve (modes_resolve.cpp) --------------------------------
 struct ResolveState {
     uint32_t icao[1024];         // dump1090.c:335: address per slot (TTL: never expires within a run)
@@ -142,5 +161,12 @@ void resolve_commit(MessageOut &out, ResolveScratch *scratch);
 void deliver_gpu(const modes_delivery *d, size_t n, int64_t buffer_base, MessageOut &out);
 // The order-dependent tail of decodeModesMessage + field decode for one evaluated frame.
 int finish_message(ResolveState &st, const modes_frame_eval &p, modes_message *out);
+
+// ---- C-ABI glue (modes_api.cpp) ----------------------------------------------
+// Where the context's last modes_detect_device / _host left its results on the device (its own
+// workspace; valid after modes_detect_wait until the next detect call), and its tile count.
+void detect_results(const modes_ctx *ctx, const modes_candidate **records, const modes_tile **tiles, uint32_t *n_tiles);
+// cudaStreamSynchronize, or its sleeping equivalent under modes_set_host_wait(1).
+cudaError_t wait_stream(cudaStream_t st);
 
 }  // namespace modes

@@ -18,9 +18,16 @@
 // receiver's own stream; whatever the scan finds inside the pad buffers is dropped.  The price is a
 // second scan over constant buffers (the scan runs at 2 T samples/s; the link delivers 25 G samples/s).
 //
-// The order-dependent half is the existing host resolver, one per receiver: the records of a data
-// buffer are re-based to that receiver's own stream position and replayed with its own address
-// cache.  Built on the public C ABI only (modes_detect_device / _fetch, modes_resolver_*).
+// The order-dependent half (cfg.gpu_resolve = 0) is the existing host resolver, one per receiver: the
+// records of a data buffer are re-based to that receiver's own stream position and replayed with its
+// own address cache.  With cfg.gpu_resolve = 1 the same replay runs on the device at collect, one warp
+// per receiver, each receiver's address cache resident in HBM between batches (launch_pool_resolve,
+// modes_resolve_gpu.cu); only the 40-byte records of the delivered messages and 36 bytes of counts and
+// statistics per receiver cross PCIe, and the host builds the structs.  Within a batch no receiver's
+// buffer depends on another's, so unlike the single-stream device resolve there is nothing to guess.
+// The detection runs through the public C ABI (modes_detect_device / _wait / _fetch); the host resolve
+// through modes_resolver_*; the device resolve reads the records where modes_detect_device left them
+// (modes::detect_results) and builds structs with modes::deliver_gpu.
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -34,6 +41,7 @@
 #include <vector>
 #include <cuda_runtime.h>
 #include "modes_b200.h"
+#include "modes_internal.h"
 
 namespace {
 
@@ -44,6 +52,9 @@ struct Receiver {
     modes_resolver *res = nullptr;
     int64_t buffers = 0;                       // buffers of this receiver decoded so far
     uint8_t carry[MODES_CARRY_BYTES];
+    // cfg.gpu_resolve: the statistics so far, and whether its resident cache is to be ignored (reset)
+    int64_t stats[8] = {};
+    bool fresh = true;
 };
 
 // A few persistent helper threads: run(n, f) executes f(0..n-1), f(0) on the calling thread.
@@ -124,6 +135,17 @@ struct modes_pool {
     };
     std::vector<Block> blocks;
     std::unique_ptr<Crew> crew;
+    // cfg.gpu_resolve: the device resolve's memory, used by one collect at a time
+    struct Device {
+        uint32_t *caches = nullptr;            // [n_receivers][1024]
+        uint32_t *work = nullptr;              // ids [max_batch], offsets [max_batch + 1], flags [4], then n_deliv [n] + stats [n][8]
+        uint32_t *h_work = nullptr;            // pinned: ids [max_batch], then n_deliv [n] + stats [n][8]
+        modes::modes_delivery *out = nullptr;  // [out_cap]
+        modes::modes_delivery *h_out = nullptr;   // pinned [out_cap]
+        size_t out_cap = 0;
+        std::vector<modes_message> spill;      // structs that do not fit the output array, for the sink
+        std::vector<size_t> first;             // [n + 1] where entry i's deliveries start
+    } dev;
     // optional caller-owned output array (modes_pool_set_output)
     modes_message *out = nullptr; uint32_t *out_rx = nullptr; size_t out_cap = 0, out_count = 0;
 };
@@ -172,6 +194,113 @@ int ensure_device(modes_pool *p) {
         if (!sl.d_batch || !sl.h_carry) return fail(p, "out of memory for %zu receivers per batch", p->max_batch);
         if (modes_device_memset(sl.d_batch, 127, bytes)) return fail(p, "device memset failed");      // dump1090.c:344 no signal
     }
+    if (p->cfg.gpu_resolve) {
+        // no clearing: every receiver starts fresh, and its first batch writes its whole cache
+        modes_pool::Device &d = p->dev;
+        const size_t mb = p->max_batch;
+        if (cudaMalloc(&d.caches, p->rx.size() * 1024 * sizeof(uint32_t)) != cudaSuccess ||
+            cudaMalloc(&d.work, (2 * mb + 5 + 9 * mb) * sizeof(uint32_t)) != cudaSuccess ||
+            cudaMallocHost(&d.h_work, 10 * mb * sizeof(uint32_t)) != cudaSuccess)
+            return fail(p, "out of memory for the device resolve of %zu receivers", p->rx.size());
+    }
+    return 0;
+}
+
+// Blocks of the receiver list for the host threads: one block of 16 or more receivers per thread.
+size_t blocks_for(size_t n) {
+    size_t n_blocks = pool_threads();
+    if (n_blocks > (n + 15) / 16) n_blocks = (n + 15) / 16;
+    return n_blocks < 1 ? 1 : n_blocks;
+}
+
+// cfg.gpu_resolve: the verdicts of the collected batch in slot `sl` (its records are where
+// modes_detect_device left them) on the device, then the structs on the host, handed over in list order.
+int resolve_on_device(modes_pool *p, const modes_pool::Slot &sl, uint64_t n_cand, modes_pool_sink_fn sink, void *user) {
+    modes_pool::Device &d = p->dev;
+    const uint32_t *ids = sl.ids.data();
+    const size_t n = sl.ids.size(), mb = p->max_batch;
+    cudaStream_t st = static_cast<cudaStream_t>(modes_stream(sl.ctx));
+    const size_t cap = 2 * (n_cand ? n_cand : 1);                  // a candidate delivers at most two messages
+    if (d.out_cap < cap) {
+        cudaFree(d.out); cudaFreeHost(d.h_out); d.out = nullptr; d.h_out = nullptr; d.out_cap = 0;
+        const size_t c = cap + cap / 2;
+        if (cudaMalloc(&d.out, c * sizeof(modes::modes_delivery)) != cudaSuccess ||
+            cudaMallocHost(&d.h_out, c * sizeof(modes::modes_delivery)) != cudaSuccess)
+            return fail(p, "out of memory for %zu deliveries", c);
+        d.out_cap = c;
+    }
+    for (size_t i = 0; i < n; i++) {
+        Receiver &r = p->rx[ids[i]];
+        d.h_work[i] = ids[i] | (r.fresh ? modes::kPoolFresh : 0u);
+        r.fresh = false;
+    }
+    modes::PoolResolve pr;
+    pr.caches = d.caches;
+    pr.ids = d.work;
+    pr.offsets = d.work + mb;
+    pr.flags = d.work + 2 * mb + 1;
+    pr.n_deliv = d.work + 2 * mb + 5;
+    pr.stats = pr.n_deliv + n;
+    pr.out = d.out;
+    pr.capacity = (uint32_t)cap;
+    const modes_candidate *records; const modes_tile *tiles; uint32_t n_tiles;
+    modes::detect_results(sl.ctx, &records, &tiles, &n_tiles);
+    uint32_t *h_counts = d.h_work + mb, *h_stats = h_counts + n;
+    cudaError_t e = cudaSetDevice(p->cfg.device);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d.work, d.h_work, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) {
+        modes::launch_pool_resolve(pr, records, tiles, n_tiles, (uint32_t)n, p->cfg.check_crc, st);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(h_counts, pr.n_deliv, 9 * n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = modes::wait_stream(st);
+    if (e != cudaSuccess) return fail(p, "device resolve failed: %s", cudaGetErrorString(e));
+    d.first.resize(n + 1);
+    d.first[0] = 0;
+    for (size_t i = 0; i < n; i++) d.first[i + 1] = d.first[i] + h_counts[i];
+    const size_t total = d.first[n];
+    if (total) {
+        e = cudaMemcpyAsync(d.h_out, d.out, total * sizeof(modes::modes_delivery), cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = modes::wait_stream(st);
+        if (e != cudaSuccess) return fail(p, "delivery download failed: %s", cudaGetErrorString(e));
+    }
+    for (size_t i = 0; i < n; i++) {
+        Receiver &r = p->rx[ids[i]];
+        for (int k = 0; k < 8; k++) r.stats[k] += h_stats[8 * i + k];
+    }
+    // The structs, receiver by receiver (each from its own stream position), one block of receivers per
+    // host thread: into the caller's array where they fit, into `spill` where the sink needs the rest.
+    const size_t base = p->out_count, out_cap = p->out ? p->out_cap : 0;
+    const size_t fit = base >= out_cap ? 0 : (total < out_cap - base ? total : out_cap - base);
+    if (sink && d.spill.size() < total - fit) d.spill.resize(total - fit);
+    const size_t n_blocks = blocks_for(n);
+    auto build = [&](size_t b) {
+        for (size_t i = n * b / n_blocks; i < n * (b + 1) / n_blocks; i++) {
+            const int64_t buffers = p->rx[ids[i]].buffers;
+            const size_t f0 = d.first[i], f1 = d.first[i + 1], in_array = f1 < fit ? f1 : (f0 < fit ? fit : f0);
+            if (in_array > f0) {
+                modes::MessageOut mo;
+                mo.array = p->out + base; mo.capacity = fit; mo.count = f0;
+                modes::deliver_gpu(d.h_out + f0, in_array - f0, buffers, mo);
+                for (size_t k = f0; k < in_array; k++) p->out_rx[base + k] = ids[i];
+            }
+            if (sink && f1 > in_array) {
+                modes::MessageOut mo;
+                mo.array = d.spill.data(); mo.capacity = total - fit; mo.count = in_array - fit;
+                modes::deliver_gpu(d.h_out + in_array, f1 - in_array, buffers, mo);
+            }
+        }
+    };
+    if (p->out || sink) {
+        if (!p->crew) p->crew.reset(new Crew(pool_threads() - 1));
+        p->crew->run(n_blocks, build);
+    }
+    if (p->out) p->out_count += total;
+    if (sink)
+        for (size_t i = 0; i < n; i++)
+            for (size_t k = d.first[i]; k < d.first[i + 1]; k++)
+                sink(user, ids[i], k < fit ? &p->out[base + k] : &d.spill[k - fit]);
+    for (size_t i = 0; i < n; i++) p->rx[ids[i]].buffers++;
     return 0;
 }
 
@@ -201,6 +330,10 @@ void modes_pool_destroy(modes_pool *p) {
         if (sl.h_carry) modes_host_free(sl.h_carry);
         if (sl.ctx) modes_destroy(sl.ctx);
     }
+    if (p->dev.caches) cudaFree(p->dev.caches);
+    if (p->dev.work) cudaFree(p->dev.work);
+    if (p->dev.h_work) cudaFreeHost(p->dev.h_work);
+    if (p->dev.out) { cudaFree(p->dev.out); cudaFreeHost(p->dev.h_out); }
     delete p;
 }
 
@@ -209,6 +342,9 @@ const char *modes_pool_last_error(const modes_pool *p) { return p ? p->err.c_str
 int modes_pool_resolve(modes_pool *p, const uint32_t *receivers, size_t n, const modes_candidate *candidates,
                        const modes_tile *tiles, modes_pool_sink_fn sink, void *user) {
     if (!p) return -1;
+    if (p->cfg.gpu_resolve)
+        return fail(p, "this pool resolves on the device (gpu_resolve = 1): its address caches live there, "
+                       "so modes_pool_resolve (the host half of a gpu_resolve = 0 pool) is not available");
     if (check_ids(p, receivers, n)) return -1;
     if (!n) return 0;
     if (!tiles) return fail(p, "no tile table");
@@ -216,9 +352,7 @@ int modes_pool_resolve(modes_pool *p, const uint32_t *receivers, size_t n, const
     const size_t n_local = modes_tile_count(1);
     // Receivers are independent: the list is cut into blocks, one host thread each; a block's messages
     // land in its own array and are moved to the caller's array / handed to the sink in list order.
-    size_t n_blocks = pool_threads();
-    if (n_blocks > (n + 15) / 16) n_blocks = (n + 15) / 16;
-    if (n_blocks < 1) n_blocks = 1;
+    const size_t n_blocks = blocks_for(n);
     if (p->blocks.size() < n_blocks) p->blocks.resize(n_blocks);
     auto tile_range = [&](size_t i, size_t &g0, size_t &g1) {
         // the data buffer of pair i is buffer 2i+1 of the batch; a position t belongs to the tile
@@ -351,6 +485,11 @@ int modes_pool_collect(modes_pool *p, modes_pool_sink_fn sink, void *user) {
     modes_pool::Slot &sl = p->slot[p->collected & 1];
     uint64_t n_cand = 0;
     if (modes_detect_wait(sl.ctx, &n_cand)) return fail(p, "%s", modes_last_error(sl.ctx));
+    if (p->cfg.gpu_resolve) {
+        sl.busy = false;
+        p->collected++;
+        return resolve_on_device(p, sl, n_cand, sink, user);
+    }
     const size_t n = sl.ids.size();
     p->cands.resize(n_cand ? n_cand : 1);
     p->tiles.resize(modes_tile_count(2 * n));
@@ -371,6 +510,10 @@ int modes_pool_ingest(modes_pool *p, const uint32_t *receivers, const uint8_t *c
 
 int modes_pool_stats(const modes_pool *p, uint32_t receiver, modes_stats *out) {
     if (!p || receiver >= p->rx.size() || !out) return -1;
+    if (p->cfg.gpu_resolve) {
+        memcpy(out->v, p->rx[receiver].stats, sizeof(out->v));
+        return 0;
+    }
     return modes_resolver_stats(p->rx[receiver].res, out);
 }
 
@@ -379,6 +522,8 @@ int modes_pool_reset(modes_pool *p, uint32_t receiver) {
     Receiver &r = p->rx[receiver];
     r.buffers = 0;
     memset(r.carry, 127, sizeof r.carry);
+    memset(r.stats, 0, sizeof r.stats);
+    r.fresh = true;                            // its next collected batch starts from an empty cache
     return modes_resolver_reset(r.res);
 }
 

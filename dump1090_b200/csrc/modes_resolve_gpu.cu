@@ -21,6 +21,10 @@
 // 56-byte candidate records never leave the GPU (47 MB -> 17 MB per GiB of the dense capture).
 // Exactness is checked on the CPU for the algorithm (tests/test_resolve_core_host.py) and on the
 // GPU against the host resolver and the oracle (tests/test_gpu_resolve.py).
+//
+// A receiver pool (modes_pool.cpp) needs none of the guessing: its batch holds one buffer per receiver,
+// so pool_resolve_kernel replays each from that receiver's resident cache and writes the cache back
+// (count, resolve_offsets_kernel, emit); tests/test_pool_gpu_resolve.py.
 #include <cstdint>
 #include <cuda_runtime.h>
 #include "modes_internal.h"
@@ -49,12 +53,81 @@ struct WarpCache {
     }
 };
 
+// The address cache of a receiver pool's buffer: nothing to track, every buffer starts from the cache
+// its receiver really has.
+struct SharedCache {
+    uint32_t *c;                 // [1024] in shared memory
+    int lane;
+    __device__ __forceinline__ uint32_t read(uint32_t s) { return c[s]; }
+    __device__ __forceinline__ void write(uint32_t s, uint32_t a) {
+        __syncwarp();
+        if (lane == 0) c[s] = a;
+        __syncwarp();
+    }
+};
+
 __device__ __forceinline__ rcore::Attempt attempt_from_words(uint32_t e0, uint32_t e3, uint32_t e4, uint32_t e5) {
     rcore::Attempt a;
     a.meta = (e3 >> 16) | (e4 << 16);                   // msgtype, flags, errorbit, nfixed
     a.crc = e5;
     a.addr = __byte_perm(e0, 0u, 0x4123);               // msg[1] << 16 | msg[2] << 8 | msg[3]
     return a;
+}
+
+// One warp replays the candidates of buffer b of the batch (t >> 17 == b) in stream order and returns
+// its delivery count.  kEmit: the deliveries are also written from out + out_base on (below `capacity`),
+// with position t - t_shift.
+template <bool kEmit, class Cache>
+__device__ __forceinline__ uint32_t replay_buffer(Cache &wc, rcore::BufferState &st, const modes_candidate *__restrict__ records,
+                                                  const modes_tile *__restrict__ tiles, uint32_t n_tiles, uint32_t b, int check_crc,
+                                                  int lane, modes_delivery *out, uint32_t out_base, uint32_t capacity, uint64_t t_shift) {
+    uint32_t n_out = 0;
+    const uint64_t v_lo = (uint64_t)b * kBufSamples + 2, v_hi = (uint64_t)(b + 1) * kBufSamples + 1;
+    uint32_t t_lo = (uint32_t)(v_lo / kTileSamples), t_hi = (uint32_t)(v_hi / kTileSamples);
+    if (t_hi >= n_tiles) t_hi = n_tiles - 1;
+    for (uint32_t ti = t_lo; ti <= t_hi; ti++) {
+        const modes_tile tl = tiles[ti];
+        for (uint32_t i0 = 0; i0 < tl.count; i0 += 32) {
+            const uint32_t n_here = min(32u, tl.count - i0);
+            // lane i holds candidate i0 + i of the tile: 14 words
+            uint32_t w[14];
+            if ((uint32_t)lane < n_here) {
+                const uint2 *rp = reinterpret_cast<const uint2 *>(records + tl.offset + i0 + lane);
+#pragma unroll
+                for (int k = 0; k < 7; k++) { const uint2 v = rp[k]; w[2 * k] = v.x; w[2 * k + 1] = v.y; }
+            } else {
+#pragma unroll
+                for (int k = 0; k < 14; k++) w[k] = 0;
+            }
+            for (uint32_t i = 0; i < n_here; i++) {
+                const uint32_t t0 = __shfl_sync(0xffffffffu, w[0], i), t1 = __shfl_sync(0xffffffffu, w[1], i);
+                const uint64_t t = ((uint64_t)t1 << 32) | t0;
+                if ((t >> 17) != (uint64_t)b) continue;            // the tile straddles a buffer boundary
+                const rcore::Attempt p1 = attempt_from_words(__shfl_sync(0xffffffffu, w[2], i), __shfl_sync(0xffffffffu, w[5], i),
+                                                             __shfl_sync(0xffffffffu, w[6], i), __shfl_sync(0xffffffffu, w[7], i));
+                const rcore::Attempt p2 = attempt_from_words(__shfl_sync(0xffffffffu, w[8], i), __shfl_sync(0xffffffffu, w[11], i),
+                                                             __shfl_sync(0xffffffffu, w[12], i), __shfl_sync(0xffffffffu, w[13], i));
+                rcore::Decision d[2];
+                rcore::candidate(st, wc, (uint32_t)(t0 & (kBufSamples - 1)), p1, p2, check_crc, d);
+#pragma unroll
+                for (int p = 0; p < 2; p++) {
+                    if (!d[p].deliver) continue;
+                    if (kEmit && lane == (int)i && out_base + n_out < capacity) {
+                        modes_delivery *o = out + out_base + n_out;
+                        uint32_t *ow = reinterpret_cast<uint32_t *>(o);
+                        const uint64_t tp = (((uint64_t)w[1] << 32) | w[0]) - t_shift;     // this lane's own t
+                        ow[0] = (uint32_t)tp; ow[1] = (uint32_t)(tp >> 32);
+#pragma unroll
+                        for (int k = 0; k < 6; k++) ow[2 + k] = w[2 + 6 * p + k];
+                        ow[8] = d[p].extra;
+                        ow[9] = d[p].crcok | (d[p].phase_corrected << 8) | (d[p].extra_is_ap << 16);
+                    }
+                    n_out++;
+                }
+            }
+        }
+    }
+    return n_out;
 }
 
 __global__ void __launch_bounds__(256)
@@ -87,53 +160,8 @@ resolve_replay_kernel(GpuResolve g, const modes_candidate *__restrict__ records,
         st.next_j = 0;
 #pragma unroll
         for (int k = 0; k < 8; k++) st.stats[k] = 0;
-        uint32_t n_out = 0;
         const uint32_t out_base = kEmit ? g.offsets[b] : 0u;
-
-        const uint64_t v_lo = (uint64_t)b * kBufSamples + 2, v_hi = (uint64_t)(b + 1) * kBufSamples + 1;
-        uint32_t t_lo = (uint32_t)(v_lo / kTileSamples), t_hi = (uint32_t)(v_hi / kTileSamples);
-        if (t_hi >= n_tiles) t_hi = n_tiles - 1;
-        for (uint32_t ti = t_lo; ti <= t_hi; ti++) {
-            const modes_tile tl = tiles[ti];
-            for (uint32_t i0 = 0; i0 < tl.count; i0 += 32) {
-                const uint32_t n_here = min(32u, tl.count - i0);
-                // lane i holds candidate i0 + i of the tile: 14 words
-                uint32_t w[14];
-                if ((uint32_t)lane < n_here) {
-                    const uint2 *rp = reinterpret_cast<const uint2 *>(records + tl.offset + i0 + lane);
-#pragma unroll
-                    for (int k = 0; k < 7; k++) { const uint2 v = rp[k]; w[2 * k] = v.x; w[2 * k + 1] = v.y; }
-                } else {
-#pragma unroll
-                    for (int k = 0; k < 14; k++) w[k] = 0;
-                }
-                for (uint32_t i = 0; i < n_here; i++) {
-                    const uint32_t t0 = __shfl_sync(0xffffffffu, w[0], i), t1 = __shfl_sync(0xffffffffu, w[1], i);
-                    const uint64_t t = ((uint64_t)t1 << 32) | t0;
-                    if ((t >> 17) != (uint64_t)b) continue;            // the tile straddles a buffer boundary
-                    const rcore::Attempt p1 = attempt_from_words(__shfl_sync(0xffffffffu, w[2], i), __shfl_sync(0xffffffffu, w[5], i),
-                                                                 __shfl_sync(0xffffffffu, w[6], i), __shfl_sync(0xffffffffu, w[7], i));
-                    const rcore::Attempt p2 = attempt_from_words(__shfl_sync(0xffffffffu, w[8], i), __shfl_sync(0xffffffffu, w[11], i),
-                                                                 __shfl_sync(0xffffffffu, w[12], i), __shfl_sync(0xffffffffu, w[13], i));
-                    rcore::Decision d[2];
-                    rcore::candidate(st, wc, (uint32_t)(t0 & (kBufSamples - 1)), p1, p2, check_crc, d);
-#pragma unroll
-                    for (int p = 0; p < 2; p++) {
-                        if (!d[p].deliver) continue;
-                        if (kEmit && lane == (int)i && out_base + n_out < g.capacity) {
-                            modes_delivery *o = g.out + out_base + n_out;
-                            uint32_t *ow = reinterpret_cast<uint32_t *>(o);
-                            ow[0] = w[0]; ow[1] = w[1];
-#pragma unroll
-                            for (int k = 0; k < 6; k++) ow[2 + k] = w[2 + 6 * p + k];
-                            ow[8] = d[p].extra;
-                            ow[9] = d[p].crcok | (d[p].phase_corrected << 8) | (d[p].extra_is_ap << 16);
-                        }
-                        n_out++;
-                    }
-                }
-            }
-        }
+        const uint32_t n_out = replay_buffer<kEmit>(wc, st, records, tiles, n_tiles, b, check_crc, lane, g.out, out_base, g.capacity, 0);
         __syncwarp();
         if (!kEmit) {
 #pragma unroll
@@ -198,6 +226,46 @@ resolve_offsets_kernel(GpuResolve g, uint32_t n_buffers, uint32_t capacity) {
     }
 }
 
+// Receiver pool: one warp per list entry i replays data buffer 2i+1 from its receiver's cache.
+// kEmit = false counts the deliveries and leaves the cache alone; kEmit = true writes the deliveries
+// at offsets[i], the statistics, and the cache back.
+template <bool kEmit>
+__global__ void __launch_bounds__(32 * kWarpsPerCta)
+pool_resolve_kernel(PoolResolve p, const modes_candidate *__restrict__ records, const modes_tile *__restrict__ tiles,
+                    uint32_t n_tiles, uint32_t n, int check_crc) {
+    __shared__ __align__(16) uint32_t s_cache[kWarpsPerCta][1024];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint32_t i = blockIdx.x * kWarpsPerCta + warp;
+    if (i >= n) return;                                                // the whole warp
+    const uint32_t id = p.ids[i] & ~kPoolFresh;
+    const bool fresh = p.ids[i] & kPoolFresh;
+    uint32_t *cache = s_cache[warp];
+    uint4 *resident = reinterpret_cast<uint4 *>(p.caches + (size_t)id * 1024);
+#pragma unroll
+    for (int k = 0; k < 8; k++)
+        reinterpret_cast<uint4 *>(cache)[32 * k + lane] = fresh ? make_uint4(0, 0, 0, 0) : resident[32 * k + lane];
+    __syncwarp();
+    SharedCache sc{cache, lane};
+    rcore::BufferState st;
+    st.next_j = 0;
+#pragma unroll
+    for (int k = 0; k < 8; k++) st.stats[k] = 0;
+    const uint32_t b = 2 * i + 1;
+    const uint32_t n_out = replay_buffer<kEmit>(sc, st, records, tiles, n_tiles, b, check_crc, lane, p.out,
+                                                kEmit ? p.offsets[i] : 0u, p.capacity, (uint64_t)b * kBufSamples);
+    if (!kEmit) {
+        if (lane == 0) p.n_deliv[i] = n_out;
+        return;
+    }
+    __syncwarp();
+#pragma unroll
+    for (int k = 0; k < 8; k++) resident[32 * k + lane] = reinterpret_cast<const uint4 *>(cache)[32 * k + lane];
+    if (lane == 0) {                                                   // p.stats is only 4-byte aligned
+#pragma unroll
+        for (int k = 0; k < 8; k++) p.stats[(size_t)i * 8 + k] = st.stats[k];
+    }
+}
+
 }  // namespace
 
 void launch_gpu_resolve(const GpuResolve &g, const modes_candidate *records, const modes_tile *tiles, uint32_t n_tiles,
@@ -213,6 +281,16 @@ void launch_gpu_resolve(const GpuResolve &g, const modes_candidate *records, con
     }
     resolve_offsets_kernel<<<1, 1024, 0, stream>>>(g, n_buffers, g.capacity);
     resolve_replay_kernel<true><<<grid, 32 * kWarpsPerCta, 0, stream>>>(g, records, tiles, n_tiles, n_buffers, check_crc);
+}
+
+void launch_pool_resolve(const PoolResolve &p, const modes_candidate *records, const modes_tile *tiles, uint32_t n_tiles,
+                         uint32_t n, int check_crc, cudaStream_t stream) {
+    const uint32_t grid = (n + kWarpsPerCta - 1) / kWarpsPerCta;
+    pool_resolve_kernel<false><<<grid, 32 * kWarpsPerCta, 0, stream>>>(p, records, tiles, n_tiles, n, check_crc);
+    GpuResolve g{};                                                    // the fields resolve_offsets_kernel uses
+    g.n_deliv = p.n_deliv; g.offsets = p.offsets; g.flags = p.flags;
+    resolve_offsets_kernel<<<1, 1024, 0, stream>>>(g, n, p.capacity);
+    pool_resolve_kernel<true><<<grid, 32 * kWarpsPerCta, 0, stream>>>(p, records, tiles, n_tiles, n, check_crc);
 }
 
 }  // namespace modes

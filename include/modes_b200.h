@@ -68,7 +68,9 @@ typedef struct modes_config {
                                    4) — and only 40-byte records of the delivered messages cross PCIe; the host
                                    builds the struct fields.  Same messages, same statistics.  Streaming decode
                                    on one GPU only; a batch denser than one candidate per 64 samples is an error
-                                   in this mode. */
+                                   in this mode.  A receiver pool (modes_pool_*) with gpu_resolve = 1 resolves on
+                                   the device too: one warp per receiver, every receiver's address cache kept in
+                                   device memory between batches; there a dense batch is repeated as usual. */
 } modes_config;
 
 /* Replaces struct modesMessage (dump1090.c:211-260): same field names and
@@ -352,7 +354,13 @@ size_t modes_tile_count(size_t n_buffers);
  * whose tail is that receiver's carry, so the kernels are the single-stream ones).  Messages of a
  * receiver are delivered in its stream order with sample_pos counted in its own stream; receivers are
  * served in the order they are listed.  Every receiver's output equals a modes_ctx fed that receiver's
- * buffers alone. */
+ * buffers alone.
+ * cfg->gpu_resolve = 0 (default): each receiver's buffer is resolved on the host, by that receiver's own
+ * modes_resolver, on MODES_POOL_THREADS threads (default 4).  cfg->gpu_resolve = 1: modes_pool_collect
+ * resolves on the device, one warp per receiver, each receiver's address cache resident in device memory
+ * (4 KiB per receiver); only the delivered messages' 40-byte records cross PCIe, and the host builds the
+ * structs.  The output (messages, order, fields, sample_pos, receiver_of, statistics, buffers) is the same
+ * byte for byte.  cfg->n_gpus is ignored: a pool uses `device` alone. */
 typedef struct modes_pool modes_pool;
 typedef void (*modes_pool_sink_fn)(void *user, uint32_t receiver, const modes_message *mm);
 /* max_batch_receivers: most receivers one modes_pool_ingest call names (0: n_receivers); sizes the
@@ -373,7 +381,8 @@ int  modes_pool_submit(modes_pool *p, const uint32_t *receivers, const uint8_t *
 int  modes_pool_collect(modes_pool *p, modes_pool_sink_fn sink, void *user);
 /* The host half alone, for candidate records produced elsewhere over a batch laid out as the pool lays
  * it out: buffer 2i = pad buffer of receivers[i] (no signal, last MODES_CARRY_BYTES = its carry), buffer
- * 2i+1 = its new buffer; candidates/tiles as modes_detect_fetch returns them for those 2n buffers. */
+ * 2i+1 = its new buffer; candidates/tiles as modes_detect_fetch returns them for those 2n buffers.
+ * Fails on a pool created with gpu_resolve = 1, whose address caches live on the device. */
 int  modes_pool_resolve(modes_pool *p, const uint32_t *receivers, size_t n, const modes_candidate *candidates,
                         const modes_tile *tiles, modes_pool_sink_fn sink, void *user);
 /* Like modes_set_output: messages are ALSO written to a caller-owned array, all receivers' in delivery
